@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — EI evaluations / second + GP fit time on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--m M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--m M] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1] / SURVEY.md section 8d "C2"): GP posterior with N = 4096
 training points, D = 16, amp * ARD Matern-5/2, fp64, synthetic seeded data; one *step* scores a
@@ -20,6 +20,10 @@ Our arm (default)
           is exchanged by libgpk.so itself (NCCL bound behind the C ABI; torch.distributed only launches the processes,
           ships the 128-byte NCCL id and reduces the timings).  Outside the timed region rank 0 scores the FULL list on
           one GPU and the merged (value, global index) must equal that arg-max: "argmax_check".
+  --dump-outputs DIR  rank 0 writes what the timed paths returned in their last step, float64: DIR/argmax.npy = the
+          merged (EI value, global candidate index) of the device path, DIR/ei_values.npy = the EI values of the rank's
+          shard that EI(model).compute returned on the e2e path.  Inputs are seeded, so two builds run with the same
+          arguments can be compared output for output.
   configs.c3  BASELINE.json configs[2] (2^20 candidates, N = 1024, D = 8) STRONG scaling: the 2^20 candidates are
           split over the ranks; wall time of one whole maximisation including the replicated fit, from a pageable
           host array and from on-device Philox candidates.
@@ -448,6 +452,9 @@ def run_ours(args, rank, world, local_rank):
     launches = tim["launches_total"] - launches0
     value = M_total * args.steps / (ms * 1e-3)
     merged = unpack_pair(d_best)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "argmax.npy"), np.array(merged, dtype=np.float64))
 
     # ---- roofline of the dominant kernel (variance GEMM), measured live with CUDA events ----
     # algorithmic flops per launch: every candidate row of the chunk contracts with the lower
@@ -478,8 +485,11 @@ def run_ours(args, rank, world, local_rank):
     acq = EI(model)
     X_shard = np.array(Xs_all[lo:hi], copy=True)      # plain (pageable) numpy array, as a RoBO maximizer would hold
 
+    last_vals = [None]
+
     def step_e2e():
         vals = acq.compute(X_shard)                   # H2D of the shard, scoring, D2H of M values (blocking)
+        last_vals[0] = vals
         i = int(np.argmax(vals))                      # random_sampling.py:50
         if world > 1:
             return mh.comm_argmax_pair(vals[i], lo + i)
@@ -498,6 +508,8 @@ def run_ours(args, rank, world, local_rank):
     ms_e2e = max_over_ranks(e0.elapsed_time(e1))
     e2e_value = M_total * args.steps / (ms_e2e * 1e-3)
     e2e_ok = bool(e2e_res[1] == merged[1] and abs(e2e_res[0] - merged[0]) <= 1e-12 * abs(merged[0]))
+    if args.dump_outputs and rank == 0:
+        np.save(os.path.join(args.dump_outputs, "ei_values.npy"), np.asarray(last_vals[0], dtype=np.float64))
 
     # second key: the round-1 figure (pinned host candidates, arg-max only: 24 bytes back)
     Xs_pinned = torch.from_numpy(X_shard).pin_memory()
@@ -647,7 +659,13 @@ def main():
     ap.add_argument("--chunk", type=int, default=16384)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c3", action="store_true", help="skip the configs[2] strong-scaling block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,114 +1,127 @@
 """Drop-in boundary, CPU side: the UNMODIFIED reference (solver, fmin facade, maximizers, its own
-GaussianProcess / GaussianProcessMCMC / MarginalizationGPMCMC classes from /root/reference) runs on top
-of the robo_b200 host layer.  libgpk.so cannot execute here (no GPU), so ``_lib.Handle`` is replaced by
-tests/fake_gpk.FakeHandle (oracle arithmetic, same method surface); the GPU suite covers the same
-surface against the real library.  Skipped where the reference tree is absent (the GPU box)."""
+GaussianProcess / GaussianProcessMCMC / FabolasGP classes) on top of the robo_b200 host layer.
+
+The reference drives robo_b200 through the ``george`` and ``emcee`` shims of robo_b200.compat.  Its calls into them,
+with their answers, were recorded by oracle/make_dropin_golden.py (tests/golden/dropin_*.npz; tests/dropin_trace.py);
+these tests issue the same calls to the shims of this tree and require the same answers, so the reference would take
+the same path through them as it did when it was recorded.  libgpk.so cannot execute without a GPU, so ``_lib.Handle``
+is replaced by tests/fake_gpk.FakeHandle (oracle arithmetic, same method surface); the GPU suite covers the same
+surface against the real library."""
 import os
-import sys
 
 import numpy as np
 import pytest
 
-REF = os.environ.get("ROBO_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "robo")), reason="reference tree not present")
-
-
-def branin(x):
-    x1, x2 = x[0], x[1]
-    return (x2 - 5.1 / (4 * np.pi ** 2) * x1 ** 2 + 5 / np.pi * x1 - 6) ** 2 + 10 * (1 - 1 / (8 * np.pi)) * np.cos(x1) + 10
+from tests import dropin_trace
 
 
 @pytest.fixture
-def reference(monkeypatch):
+def fake(monkeypatch):
     from tests import fake_gpk
-    fake_gpk.install(monkeypatch)
-    from robo_b200 import compat
-    saved = {k: sys.modules.get(k) for k in list(sys.modules) if k.split(".")[0] in ("george", "emcee", "pybnn", "pyrfr", "robo")}
-    for k in list(sys.modules):
-        if k.split(".")[0] in ("george", "robo"):
-            del sys.modules[k]
-    compat.install(force_emcee=True)
-    monkeypatch.syspath_prepend(REF)
-    yield
-    for k in list(sys.modules):
-        if k.split(".")[0] in ("george", "emcee", "pybnn", "pyrfr", "robo"):
-            del sys.modules[k]
-    for k, v in saved.items():
-        if v is not None:
-            sys.modules[k] = v
+    return fake_gpk.install(monkeypatch)
 
 
-def test_reference_solver_drives_robo_b200_objects(reference):
-    """test/test_solver/test_bayesian_optimization.py:28-49 with the product's model / acquisition /
-    maximizer handed to the reference's own BayesianOptimization solver."""
-    from robo.solver.bayesian_optimization import BayesianOptimization
+def branin_kernel():
+    from robo_b200 import kernels as K
+    return 2 * K.Matern52Kernel(np.ones(2), ndim=2)                # robo/fmin/bayesian_optimization.py:75-81
+
+
+def fabolas_kernel():
+    from robo_b200 import kernels as K
+    k = 1.3 * K.Matern52Kernel(np.ones(1) * 0.4, ndim=3, axes=0)
+    k *= K.Matern52Kernel(np.ones(1) * 0.6, ndim=3, axes=1)
+    k *= K.Matern52Kernel(np.ones(1) * 0.9, ndim=3, axes=2)
+    return k
+
+
+KERNELS = {"branin": branin_kernel, "fabolas": fabolas_kernel}
+
+
+def replay_matches(golden_dir, scenario):
+    """Every recorded call gives the recorded answer (LinAlgError where the reference met one).  Returns the number
+    of calls checked and the scenario's stored results."""
+    path = os.path.join(golden_dir, scenario + ".npz")
+    n = 0
+    for i, op, rec, got in dropin_trace.replay(path, KERNELS):
+        assert set(rec) == set(got), (i, op["op"])
+        for k in rec:
+            r, g = np.asarray(rec[k], dtype=np.float64), np.asarray(got[k], dtype=np.float64)
+            assert r.shape == g.shape, (i, op["op"], k)
+            scale = np.max(np.abs(r[np.isfinite(r)]), initial=1.0)
+            np.testing.assert_allclose(g, r, rtol=1e-9, atol=1e-12 * scale, err_msg="call %d (%s) %s" % (i, op["op"], k))
+        n += 1
+    return n, dropin_trace.load(path)[1]
+
+
+def test_reference_solver_drives_robo_b200_objects(fake, golden_dir):
+    """test/test_solver/test_bayesian_optimization.py:28-49: the reference's own BayesianOptimization solver drove the
+    product's model / acquisition / maximizer; its recorded calls (train, update, maximize) on fresh objects give the
+    recorded next points."""
     from robo_b200 import kernels as K
     from robo_b200.acquisition_functions import LCB
     from robo_b200.maximizers import RandomSampling
     from robo_b200.models import GaussianProcess
+    ops, ref = dropin_trace.load(os.path.join(golden_dir, "dropin_solver.npz"))
     lower, upper = np.zeros(1), np.ones(1) * 6
-    model = GaussianProcess(K.Matern52Kernel(np.ones(1), ndim=1), noise=1e-3, lower=lower, upper=upper)
+    model = GaussianProcess(K.Matern52Kernel(np.ones(1), ndim=1), noise=1e-3, lower=lower, upper=upper,
+                            rng=np.random.RandomState(2))
     acq = LCB(model)
-    solver = BayesianOptimization(lambda x: np.sin(3 * x[0]) * 4 * (x[0] - 1) * (x[0] + 2), lower, upper, acq, model,
-                                  RandomSampling(acq, lower, upper), rng=np.random.RandomState(0))
-    inc, inc_val = solver.run(num_iterations=6)
-    assert len(solver.incumbents) == 6 and len(solver.incumbents_values) == 6 and len(solver.time_overhead) == 6
-    assert np.all(np.array(inc) >= lower) and np.all(np.array(inc) <= upper)
-    assert model.gp.handle.n_fits > 3
+    maximizer = RandomSampling(acq, lower, upper, rng=np.random.RandomState(1))
+    assert [op["op"] for op in ops] == ["train", "update", "maximize"] * 3
+    state = np.random.get_state()
+    np.random.seed(7)                       # RandomSampling draws its candidates from numpy's global generator
+    try:
+        for op in ops:
+            arr = op["arrays"]
+            if op["op"] == "train":
+                model.train(arr["arg0"], arr["arg1"], **op["kw"])
+            elif op["op"] == "update":
+                acq.update(model)
+            else:
+                x = maximizer.maximize()
+                assert np.all(x >= lower) and np.all(x <= upper)
+                np.testing.assert_allclose(x, arr["out"], rtol=1e-9, atol=1e-12)
+    finally:
+        np.random.set_state(state)
+    assert len(ref["incumbents"]) == 6 and len(ref["incumbents_values"]) == 6
+    assert model.gp.handle.n_fits >= 3
 
 
 @pytest.mark.parametrize("maximizer", ["random", "scipy", "differential_evolution"])
-def test_unmodified_reference_fmin_gp(reference, maximizer):
+def test_unmodified_reference_fmin_gp(fake, golden_dir, maximizer):
     """robo.fmin.bayesian_optimization (reference facade + solver + maximizers + the reference's own
     GaussianProcess class) with george replaced by the robo_b200 shim."""
-    from robo.fmin import bayesian_optimization
+    n, res = replay_matches(golden_dir, "dropin_fmin_gp_" + maximizer)
+    assert n > 100
     lower, upper = np.array([-5.0, 0.0]), np.array([10.0, 15.0])
-    res = bayesian_optimization(branin, lower, upper, num_iterations=7, maximizer=maximizer, acquisition_func="ei",
-                                model_type="gp", n_init=3, rng=np.random.RandomState(2))
-    assert len(res["y"]) == 7 and np.all(np.array(res["X"]) >= lower) and np.all(np.array(res["X"]) <= upper)
-    assert res["f_opt"] == min(res["y"])
+    assert len(res["y"]) == 7 and np.all(res["X"] >= lower) and np.all(res["X"] <= upper)
 
 
-def test_unmodified_reference_fmin_gp_mcmc_log_ei(reference):
-    """the facade's default path: GaussianProcessMCMC (reference class, emcee shim) + MarginalizationGPMCMC(LogEI)."""
-    import robo.fmin  # noqa: F401
-    facade = sys.modules["robo.fmin.bayesian_optimization"]
+def test_unmodified_reference_fmin_gp_mcmc_log_ei(fake, golden_dir):
+    """the facade's default path: GaussianProcessMCMC (reference class, emcee shim) + MarginalizationGPMCMC(LogEI),
+    with short chains (chain_length=6, burnin_steps=4)."""
+    ops = dropin_trace.load(os.path.join(golden_dir, "dropin_fmin_gp_mcmc_log_ei.npz"))[0]
+    assert sum(op["op"] == "run_mcmc" for op in ops) >= 2
+    n, res = replay_matches(golden_dir, "dropin_fmin_gp_mcmc_log_ei")
     lower, upper = np.array([-5.0, 0.0]), np.array([10.0, 15.0])
-    real = facade.GaussianProcessMCMC
-
-    def short_chains(*a, **kw):
-        kw.update(chain_length=6, burnin_steps=4)
-        return real(*a, **kw)
-    facade.GaussianProcessMCMC = short_chains
-    try:
-        res = facade.bayesian_optimization(branin, lower, upper, num_iterations=5, n_init=3, rng=np.random.RandomState(3))
-    finally:
-        facade.GaussianProcessMCMC = real
-    assert len(res["y"]) == 5 and np.all(np.array(res["X"]) >= lower) and np.all(np.array(res["X"]) <= upper)
+    assert len(res["y"]) == 5 and np.all(res["X"] >= lower) and np.all(res["X"] <= upper)
 
 
-def test_reference_gp_class_on_shim_matches_golden(reference, golden_dir):
-    """The reference's own GaussianProcess on the george shim reproduces the golden vectors that were
-    generated with the same class on the oracle: the shim is a faithful george.GP for RoBO's call pattern."""
-    import george
-    from robo.models.gaussian_process import GaussianProcess
-    from robo.acquisition_functions.ei import EI
+def test_reference_gp_class_on_shim_matches_golden(fake, golden_dir):
+    """The reference's own GaussianProcess on the george shim reproduced the golden vectors that were generated with
+    the same class on the oracle (the shim is a faithful george.GP for RoBO's call pattern), and the shim still
+    answers that call pattern the same way."""
+    replay_matches(golden_dir, "dropin_gp_class_branin_ny1")
+    ref = dropin_trace.load(os.path.join(golden_dir, "dropin_gp_class_branin_ny1.npz"))[1]
     d = np.load(os.path.join(golden_dir, "gp_branin_ny1.npz"))
-    k = 2 * george.kernels.Matern52Kernel(np.ones(2), ndim=2)
-    k.set_parameter_vector(np.array([np.log(1.7), np.log(0.15), np.log(0.4)]))
-    from robo.priors.default_priors import DefaultPrior
-    model = GaussianProcess(k, prior=DefaultPrior(len(k) + 1), noise=float(d["noise"]), normalize_input=True, normalize_output=True,
-                            lower=d["lower"], upper=d["upper"], rng=np.random.RandomState(0))
-    model.train(d["X"], d["y"], do_optimize=False)
-    mu, var = model.predict(d["Xs"])
-    np.testing.assert_allclose(mu, d["mu"], rtol=1e-9)
-    np.testing.assert_allclose(var, d["var"], rtol=1e-8)
-    np.testing.assert_allclose(EI(model).compute(d["Xs"]), d["acq_ei"], rtol=1e-7, atol=1e-12)
-    for t, ref in zip(d["nll_thetas"], d["nll_vals"]):
-        assert abs(model.nll(t) - ref) <= 1e-9 * abs(ref) or ref == 1e25
+    np.testing.assert_allclose(ref["mu"], d["mu"], rtol=1e-9)
+    np.testing.assert_allclose(ref["var"], d["var"], rtol=1e-8)
+    np.testing.assert_allclose(ref["acq_ei"], d["acq_ei"], rtol=1e-7, atol=1e-12)
+    for v, t in zip(ref["nll_vals"], d["nll_vals"]):
+        assert abs(v - t) <= 1e-9 * abs(t) or t == 1e25
 
 
-def test_product_host_layer_on_fake_handle_matches_golden(reference, golden_dir):
+def test_product_host_layer_on_fake_handle_matches_golden(fake, golden_dir):
     """robo_b200's own classes (host logic: normalisation, hypers bookkeeping, incumbent, retry, EI quirks)
     against the golden vectors, with the C library substituted by the oracle."""
     from tests.golden_cases import kernel_spec, load_case
@@ -128,45 +141,29 @@ def test_product_host_layer_on_fake_handle_matches_golden(reference, golden_dir)
             np.testing.assert_allclose(cls(model).compute(d["Xs"]), d[key], rtol=1e-6, atol=1e-10)
 
 
-def test_fabolas_subclasses_ride_the_path(reference):
-    """robo/models/fabolas_gp.py (FabolasGP, FabolasGPMCMC) UNMODIFIED on the george / emcee shims, next to the
-    product's own FabolasGP / FabolasGPMCMC (robo_b200/models/fabolas_gp.py): same predictions, since both are the
-    base classes plus the input transform of fabolas_gp.py:122-126."""
-    import george
-    from robo.models.fabolas_gp import FabolasGP as RefFabolasGP, FabolasGPMCMC as RefFabolasGPMCMC
-    from robo_b200 import kernels as K
+def test_fabolas_subclasses_ride_the_path(fake, golden_dir):
+    """robo/models/fabolas_gp.py (FabolasGP, FabolasGPMCMC) UNMODIFIED on the george / emcee shims (replayed), next to
+    the product's own FabolasGP / FabolasGPMCMC (robo_b200/models/fabolas_gp.py): same predictions as the reference
+    class gave, since both are the base classes plus the input transform of fabolas_gp.py:122-126."""
+    from oracle.make_dropin_golden import fabolas_problem
     from robo_b200.acquisition_functions import EI, MarginalizationGPMCMC
     from robo_b200.models import FabolasGP, FabolasGPMCMC
-    rng = np.random.RandomState(5)
-    lower, upper = np.array([-1.0, 2.0]), np.array([3.0, 5.0])
-    X = np.concatenate((lower + (upper - lower) * rng.rand(25, 2), rng.rand(25, 1)), axis=1)
-    y = np.sin(X[:, 0]) + 0.3 * X[:, 1] + (1 - X[:, 2]) ** 2
-    Xt = np.concatenate((lower + (upper - lower) * rng.rand(9, 2), rng.rand(9, 1)), axis=1)
+    replay_matches(golden_dir, "dropin_fabolas")
+    ref = dropin_trace.load(os.path.join(golden_dir, "dropin_fabolas.npz"))[1]
+    assert ref["mcmc_hypers"].shape == (10, 5) and ref["mcmc_mu"].shape == (9,)
+    lower, upper, X, y, Xt = fabolas_problem()
 
     def basis(s):
         return (1 - s) ** 2                                   # fabolas.py:96-98
 
-    def ref_kernel():
-        k = 1.3 * george.kernels.Matern52Kernel(np.ones(1) * 0.4, ndim=3, axes=0)
-        k *= george.kernels.Matern52Kernel(np.ones(1) * 0.6, ndim=3, axes=1)
-        k *= george.kernels.Matern52Kernel(np.ones(1) * 0.9, ndim=3, axes=2)
-        return k
-
-    def own_kernel():
-        k = 1.3 * K.Matern52Kernel(np.ones(1) * 0.4, ndim=3, axes=0)
-        k *= K.Matern52Kernel(np.ones(1) * 0.6, ndim=3, axes=1)
-        k *= K.Matern52Kernel(np.ones(1) * 0.9, ndim=3, axes=2)
-        return k
-    ref = RefFabolasGP(ref_kernel(), basis_function=basis, noise=1e-3, lower=lower, upper=upper, rng=np.random.RandomState(0))
-    own = FabolasGP(own_kernel(), basis_function=basis, noise=1e-3, lower=lower, upper=upper, rng=np.random.RandomState(0))
-    ref.train(X, y, do_optimize=False)
+    own = FabolasGP(fabolas_kernel(), basis_function=basis, noise=1e-3, lower=lower, upper=upper,
+                    rng=np.random.RandomState(0))
     own.train(X, y, do_optimize=False)
-    m1, v1 = ref.predict(Xt)
     m2, v2 = own.predict(Xt)
-    np.testing.assert_allclose(m2, m1, rtol=1e-9, atol=1e-12)
-    np.testing.assert_allclose(v2, v1, rtol=1e-7)
-    np.testing.assert_allclose(EI(own).compute(Xt), EI(ref).compute(Xt), rtol=1e-6, atol=1e-12)
-    # MCMC variants: short chains; the product's sub-models are FabolasGP on the device path and the marginalised
+    np.testing.assert_allclose(m2, ref["mu"], rtol=1e-9, atol=1e-12)
+    np.testing.assert_allclose(v2, ref["var"], rtol=1e-7)
+    np.testing.assert_allclose(EI(own).compute(Xt), ref["acq_ei"], rtol=1e-6, atol=1e-12)
+    # MCMC variant: short chains; the product's sub-models are FabolasGP on the device path and the marginalised
     # acquisition goes through the fused multi-model call on transformed inputs
     class Prior(object):
         def __init__(self, r):
@@ -177,11 +174,7 @@ def test_fabolas_subclasses_ride_the_path(reference):
 
         def sample_from_prior(self, n):
             return self.r.uniform(-2, 1, size=(n, 5))
-    refm = RefFabolasGPMCMC(ref_kernel(), basis_func=basis, prior=Prior(np.random.RandomState(1)), n_hypers=10,
-                            chain_length=4, burnin_steps=3, lower=lower, upper=upper, rng=np.random.RandomState(2))
-    refm.train(X, y, do_optimize=True)
-    assert len(refm.models) == 10 and refm.predict(Xt)[0].shape == (9,)
-    ownm = FabolasGPMCMC(own_kernel(), basis_func=basis, prior=Prior(np.random.RandomState(1)), n_hypers=10,
+    ownm = FabolasGPMCMC(fabolas_kernel(), basis_func=basis, prior=Prior(np.random.RandomState(1)), n_hypers=10,
                          chain_length=4, burnin_steps=3, lower=lower, upper=upper, rng=np.random.RandomState(2))
     ownm.train(X, y, do_optimize=True)
     assert len(ownm.models) == 10 and all(isinstance(m, FabolasGP) for m in ownm.models)

@@ -302,3 +302,24 @@ def test_sample_functions_on_device_path_uses_raw_covariance():
         np.random.seed(5)
         one = model.sample_functions(Xt, n_funcs=1)
         assert one.shape == (1, M)
+
+
+def test_bench_dump_outputs_of_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: the merged arg-max of the device path and the EI values of the e2e path, as float64
+    arrays that agree with each other and with the JSON line."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    m = 4096
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--m", str(m),
+                          "--no-c3", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900, cwd=root)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["argmax_check"] is True
+    best = np.load(os.path.join(str(tmp_path), "argmax.npy"))
+    ei = np.load(os.path.join(str(tmp_path), "ei_values.npy"))
+    assert best.dtype == ei.dtype == np.float64 and best.shape == (2,) and ei.shape == (m,)
+    assert best[0] == line["argmax"]["merged"]["value"] and int(best[1]) == line["argmax"]["merged"]["index"]
+    assert int(np.argmax(ei)) == int(best[1]) and abs(ei[int(best[1])] - best[0]) <= 1e-12 * abs(best[0])
