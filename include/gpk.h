@@ -4,6 +4,7 @@
  * point replaces a call the reference makes into george / scipy-LAPACK / scipy.stats from
  *   robo/models/gaussian_process.py          (train / nll / predict)
  *   robo/acquisition_functions/{ei,log_ei,pi,lcb}.py   (compute)
+ *   robo/acquisition_functions/information_gain{,_per_unit_cost}.py and robo/util/epmgp.py (entropy search)
  * The reference is pure Python; its "FFI" for this path is george's Cython bridge, so the
  * binding a RoBO maintainer would add is a ctypes stub (see INTEGRATION.md and
  * robo_b200/_lib.py, which is exactly that stub).
@@ -296,6 +297,32 @@ int gpk_measure_int8_peak(gpk_handle* h, double* tops);
  * random_operands = 0: constant operand pattern (no switching activity: does not reach the power limit); 1: pseudo-random
  * bytes, the statistics of real digit slices. */
 int gpk_measure_int8_peak_sustained(gpk_handle* h, double seconds, int random_operands, double* tops);
+
+/* ---- entropy search (robo/acquisition_functions/information_gain.py, robo/util/epmgp.py) ----------------------- */
+/* epmgp.joint_min(mu, V, with_derivatives=True) (epmgp.py:11-81) on caller-supplied moments: expectation propagation
+ * per representer point (sweeps in the reference's order, stop at |diff| < 1e-3 or after 50), log Z and its
+ * derivatives, then the renormalisation.  mu (nb), V (nb x nb) host arrays, 2 <= nb <= 128.  Outputs (any may be NULL):
+ * logP (nb), dlogPdMu (nb x nb), dlogPdSigma (nb x nb(nb+1)/2, lower triangle row-major per row), dlogPdMudMu
+ * (nb x nb x nb), sweeps (nb ints: EP sweeps run per point).  Uses the buffers of the handle's entropy-search state:
+ * a later gpk_es_compute needs a new gpk_es_update.  GPK_NOT_PD when I + R^T Sigma R stays indefinite after the
+ * 1e-10 / 1e-6 jitter retries (:147-153), GPK_BAD_ARG when an update yields NaN variances (:204-207). */
+int gpk_es_joint_min(gpk_handle* h, const double* mu, const double* V, int nb, double* logP, double* dlogPdMu,
+                     double* dlogPdSigma, double* dlogPdMudMu, int* sweeps);
+/* InformationGain.update after the representer points were sampled (information_gain.py:153-167): zb (nb x d) raw
+ * inputs, lmb (nb) their sampling-acquisition values, np_grid hallucinated values (Np), sn2 = model.get_noise().
+ * Runs predict(zb, full_cov=True) with its eps clip, EP, and prepares B = K^-1 k(X, zb), the packed quadratic-form
+ * operand, W = norm.ppf(linspace(1/(Np+1), 1-1/(Np+1), Np)) and the current entropy H on the device.  One state per
+ * handle.  logP_out (nb) may be NULL.  GPK_NOT_FITTED without a fit; GPK_BAD_ARG when lmb is not finite (the reference
+ * raises ValueError in compute, :207-211), nb is outside 2..128 or np_grid < 1. */
+int gpk_es_update(gpk_handle* h, const double* zb, int nb, const double* lmb, int np_grid, double sn2, double* logP_out);
+/* InformationGain.compute(X) (information_gain.py:87-125, 169-203, 253-272) for m raw candidates: out (m, may be NULL)
+ * = the change of entropy of p_min per candidate; NaN or +inf become -DBL_MAX; with lower / upper (d each, the
+ * acquisition's bounds, NULL: no rule) a candidate outside them scores np.spacing(1).  best_val / best_idx: numpy.argmax
+ * of out.  GPK_NOT_FITTED when the model was refitted after gpk_es_update. */
+int gpk_es_compute(gpk_handle* h, const double* Xs, long m, const double* lower, const double* upper, double* out,
+                   double* best_val, long* best_idx);
+/* The EP outputs of the last gpk_es_update or gpk_es_joint_min (shapes as there; any may be NULL). */
+int gpk_es_get_state(gpk_handle* h, double* logP, double* dlogPdMu, double* dlogPdSigma, double* dlogPdMudMu, int* sweeps);
 
 /* ---- introspection (tests / debugging) ----------------------------------------------- */
 int gpk_get_factor(gpk_handle* h, double* L /* n x n row-major, lower */);

@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgpk.so")
 SOURCES = ["gpk_api.cu"]
-HEADERS = ["gpk_internal.cuh", "gpk_gemm.cuh", "gpk_kernels.cuh", "gpk_diag16.cuh", "gpk_chain.cuh", "gpk_multi.inl", "gpk_ozaki.cuh", os.path.join("..", "..", "include", "gpk.h")]
+HEADERS = ["gpk_internal.cuh", "gpk_gemm.cuh", "gpk_kernels.cuh", "gpk_diag16.cuh", "gpk_chain.cuh", "gpk_multi.inl", "gpk_ozaki.cuh", "gpk_es.cuh", os.path.join("..", "..", "include", "gpk.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-shared"]
 

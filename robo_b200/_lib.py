@@ -65,6 +65,10 @@ _SIGNATURES = {
     "gpk_measure_fp64_peaks": [_vp, _dp, _dp],
     "gpk_measure_int8_peak": [_vp, _dp],
     "gpk_measure_int8_peak_sustained": [_vp, C.c_double, C.c_int, _dp],
+    "gpk_es_joint_min": [_vp, _dp, _dp, C.c_int, _dp, _dp, _dp, _dp, _ip],
+    "gpk_es_update": [_vp, _dp, C.c_int, _dp, C.c_int, C.c_double, _dp],
+    "gpk_es_compute": [_vp, _dp, C.c_long, _dp, _dp, _dp, _dp, _lp],
+    "gpk_es_get_state": [_vp, _dp, _dp, _dp, _dp, _ip],
     "gpk_get_factor": [_vp, _dp],
     "gpk_get_linv": [_vp, _dp],
     "gpk_get_z": [_vp, _dp],
@@ -401,6 +405,49 @@ class Handle(object):
         a = C.c_double()
         self._check(self.lib.gpk_measure_int8_peak_sustained(self._h, float(seconds), 1 if random_operands else 0, C.byref(a)))
         return a.value
+
+    # -- entropy search (gpk_es_*) ----------------------------------------------------------
+    def _es_out(self, nb):
+        return dict(logP=np.empty(nb), dlogPdMu=np.empty((nb, nb)), dlogPdSigma=np.empty((nb, nb * (nb + 1) // 2)),
+                    dlogPdMudMu=np.empty((nb, nb, nb)), sweeps=np.empty(nb, dtype=np.int32))
+
+    def es_joint_min(self, mu, V):
+        """epmgp.joint_min(mu, V, with_derivatives=True) on the device -> dict(logP, dlogPdMu, dlogPdSigma,
+        dlogPdMudMu, sweeps)."""
+        mu, V = f64(mu).ravel(), f64(V)
+        nb = mu.size
+        r = self._es_out(nb)
+        self._check(self.lib.gpk_es_joint_min(self._h, _as_dp(mu), _as_dp(V), nb, _as_dp(r["logP"]), _as_dp(r["dlogPdMu"]),
+                                              _as_dp(r["dlogPdSigma"]), _as_dp(r["dlogPdMudMu"]),
+                                              r["sweeps"].ctypes.data_as(_ip)))
+        return r
+
+    def es_update(self, zb, lmb, np_grid, sn2):
+        """Entropy-search state for representer points zb (raw inputs) -> logP (nb,)."""
+        zb, lmb = f64(zb), f64(lmb).ravel()
+        logP = np.empty(lmb.size)
+        self._check(self.lib.gpk_es_update(self._h, _as_dp(zb), lmb.size, _as_dp(lmb), int(np_grid), float(sn2),
+                                           _as_dp(logP)))
+        return logP
+
+    def es_compute(self, Xs, lower=None, upper=None, want_values=True):
+        """-> dict(values, best_val, best_idx) of the information gain at raw candidates Xs."""
+        Xs = f64(Xs)
+        m = Xs.shape[0]
+        out = np.empty(m) if want_values else None
+        lo = None if lower is None else f64(lower).ravel()
+        up = None if upper is None else f64(upper).ravel()
+        bv, bi = C.c_double(), C.c_long(-1)
+        self._check(self.lib.gpk_es_compute(self._h, _as_dp(Xs), m, _as_dp(lo) if lo is not None else None,
+                                            _as_dp(up) if up is not None else None,
+                                            _as_dp(out) if want_values else None, C.byref(bv), C.byref(bi)))
+        return dict(values=out, best_val=bv.value, best_idx=bi.value)
+
+    def es_get_state(self, nb):
+        r = self._es_out(nb)
+        self._check(self.lib.gpk_es_get_state(self._h, _as_dp(r["logP"]), _as_dp(r["dlogPdMu"]), _as_dp(r["dlogPdSigma"]),
+                                              _as_dp(r["dlogPdMudMu"]), r["sweeps"].ctypes.data_as(_ip)))
+        return r
 
     # -- introspection ----------------------------------------------------------------
     def get_factor(self, n):

@@ -155,6 +155,14 @@ struct gpk_handle {
     void* comm = nullptr;
     int rank = 0, world = 1;
     DevBuf gather, best_global;
+
+    // entropy search (gpk_es.cuh): one state per handle, written by gpk_es_update
+    DevBuf es_raw, es_scr, es_logP, es_dmu, es_dsig, es_dmumu, es_sweeps, es_F, es_jl, es_Bt, es_zb, es_zbop, es_W, es_lmb,
+           es_cand, es_var, es_KZ, es_S, es_bb, es_best, es_lo, es_up;
+    bool es_ready = false;
+    int es_nb = 0, es_np = 0;
+    double es_sn2 = 0.0, es_H = 0.0;
+    long es_linv_serial = -1;
 };
 
 namespace {
@@ -1141,7 +1149,10 @@ int gpk_destroy(gpk_handle* h) {
                       &h->scal, &h->status, &h->jobs, &h->cand, &h->Kstar, &h->Kstar2, &h->cand2, &h->part_mu, &h->part_ssq, &h->out_mu,
                       &h->out_var, &h->out_acq, &h->block_best, &h->best, &h->nneg, &h->Vt, &h->cov, &h->XsT,
                       &h->tmpjobs, &h->alpha, &h->tmp1, &h->tmp2, &h->tmp3, &h->chain_cnt, &h->dprof, &h->Xts, &h->tile_cnt, &h->oz_Pq, &h->oz_Kq, &h->oz_Kq2, &h->oz_eP, &h->oz_emax, &h->oz_mu, &h->oz_mu2, &h->oz_pmu2, &h->oz_scratch,
-                      &h->multi_cand, &h->multi_A, &h->multi_B, &h->multi_out, &h->multi_bb, &h->gather, &h->best_global};
+                      &h->multi_cand, &h->multi_A, &h->multi_B, &h->multi_out, &h->multi_bb, &h->gather, &h->best_global,
+                      &h->es_raw, &h->es_scr, &h->es_logP, &h->es_dmu, &h->es_dsig, &h->es_dmumu, &h->es_sweeps, &h->es_F,
+                      &h->es_jl, &h->es_Bt, &h->es_zb, &h->es_zbop, &h->es_W, &h->es_lmb, &h->es_cand, &h->es_var, &h->es_KZ,
+                      &h->es_S, &h->es_bb, &h->es_best, &h->es_lo, &h->es_up};
     for (DevBuf* b : bufs)
         if (b->p) cudaFree(b->p);
     if (h->ev_ok)
@@ -2598,3 +2609,4 @@ int gpk_get_timings(gpk_handle* h, double* out /* 16 */) {
 }  // extern "C"
 
 #include "gpk_multi.inl"
+#include "gpk_es.cuh"

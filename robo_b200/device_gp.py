@@ -252,6 +252,17 @@ class DeviceGP(object):
         self._push_cfg()
         return self.handle.acq(Xs, kind, eta, par, want_values, want_moments)
 
+    def es_update(self, zb, lmb, np_grid, sn2):
+        """Entropy-search state of this model on the device (gpk_es_update) -> logP."""
+        self._restore()
+        self._push_cfg()
+        return self.handle.es_update(zb, lmb, np_grid, sn2)
+
+    def es_compute(self, Xs, lower=None, upper=None, want_values=True):
+        self._restore()
+        self._push_cfg()
+        return self.handle.es_compute(Xs, lower, upper, want_values)
+
     def sample_conditional(self, y, t, size=1):
         mu, cov = self.posterior_cov(t)
         if size > 1:

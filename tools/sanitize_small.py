@@ -66,4 +66,17 @@ for h in hs:
 h = _lib.moments_handle()
 print(h.acq_moments(rng.randn(100), rng.rand(100) + 0.1, _lib.ACQ_LOG_EI, 0.0, 0.0)[0][:3])
 print(h.reduce_models(rng.rand(4, 50), rng.rand(4, 50))[1][:3])
+# entropy search: EP (gpk_es_ep_kernel, gpk_es_renorm_kernel), per-update prep (gpk_es_pack_kernel, gpk_es_grid_kernel,
+# gpk_es_gemm_kernel) and two scoring chunks (gpk_es_gemm_kernel, gpk_es_score_kernel)
+h = _lib.Handle(0)
+h.set_option("chunk", 256)
+h.set_data(X, y)
+h.set_input_bounds(np.zeros(D), np.ones(D))
+h.set_output_transform(True, 0.5, 2.0)
+h.set_kernel(f["family"], f["log_amp"], f["axis"], f["group"], f["log_metric"])
+h.fit(1e-3 + 1.25e-12, float(y.mean()))
+print("es logP", h.es_update(rng.rand(20, D), np.log(rng.rand(20) + 0.1), 40, 1e-3)[:3])
+r = h.es_compute(Xs[:400], np.zeros(D), np.ones(D))
+print("es best", r["best_idx"], h.es_joint_min(np.zeros(5), np.eye(5))["sweeps"])
+h.close()
 print("done")
